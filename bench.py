@@ -2,6 +2,7 @@
 """Benchmark of the detection hot path (BASELINE.json metric: images/sec).
 
   python bench.py [--gpus N] [--steps K] [--warmup W] [--workload frcnn_r50|frcnn_r101|ssd] [--impl ours|reference]
+                  [--dump-outputs DIR]
 
 A "step" = one pass of the forward hot path over one batch of synthetic images
 (N=1 workload: BASELINE.json configs[1] -- Faster R-CNN ResNet-50, COCO config,
@@ -13,8 +14,8 @@ NCCL once, every step all-gathers the padded detection records.
            on the engine's stream, max over ranks).
 `e2e`    : the same through the public host-buffer call (pinned host images ->
            H2D -> forward -> D2H of boxes/scores/labels/counts inside the timed region).
-`--impl reference`: the CPU oracle port of the reference forward (TF1 itself cannot be
-           installed here) on all host cores, one image per step (a bounded sample).
+`--impl reference`: the CPU oracle port of the reference forward (the original needs
+           TensorFlow 1) on all host cores, one image of the batch per step.
 """
 import argparse
 import json
@@ -114,6 +115,14 @@ def conv_traffic(workload):
     return None, 'not captured'
 
 
+def write_outputs(out_dir, arrays):
+    """--dump-outputs: one DIR/<name>.npy per output, floats as float32, integers as float64 (exact)."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, a in arrays.items():
+        a = np.asarray(a)
+        np.save(os.path.join(out_dir, name + '.npy'), a.astype(np.float32 if a.dtype == np.float32 else np.float64))
+
+
 def build_config(wl):
     from luminoth_b200 import default_config
     return default_config(wl['model'], wl['overrides'])
@@ -176,22 +185,21 @@ def run_reference(args, wl):
         if time.perf_counter() - t_start > budget_s / 3:
             break
     t0 = time.perf_counter()
-    done = 0
     for i in range(args.steps):
-        opredict.network_outputs(imgs[i % len(imgs)], wts, cfg)
-        done += 1
-        if time.perf_counter() - t0 > budget_s:
-            break
+        objects, labels, probs, _ = opredict.network_outputs(imgs[i % len(imgs)], wts, cfg)
     dt = time.perf_counter() - t0
-    v = done / dt
+    v = args.steps / dt
+    if args.dump_outputs:       # the engine's layout: a batch of one image, detections in the first counts[0] rows
+        write_outputs(args.dump_outputs, {'boxes': objects[None], 'scores': probs[None], 'labels': labels[None],
+                                          'counts': np.array([len(probs)])})
     line = {'impl': 'reference', 'metric': 'images/sec', 'value': v, 'unit': 'images/s', 'n_gpus': args.gpus,
-            'steps': done, 'warmup': args.warmup, 'ms_per_step': 1000.0 * dt / done, 'higher_is_better': True,
+            'steps': args.steps, 'warmup': args.warmup, 'ms_per_step': 1000.0 * dt / args.steps, 'higher_is_better': True,
             'scaling': 'weak', 'vs_baseline': None, 'dtype': 'f32', 'data': 'synthetic',
             'config': {'workload': wl['name'], 'sample': '1 image of the batch per step'},
             'cpu_baseline': {'value': v, 'unit': 'images/s', 'cores': threads, 'kind': 'port',
                              'sample': '%d images, one per step (oracle port of the reference forward; TF1 not '
                                        'installable); thread count picked as the fastest of a calibration sweep up to '
-                                       '%d host threads' % (done, os.cpu_count() or 1)},
+                                       '%d host threads' % (args.steps, os.cpu_count() or 1)},
             'e2e': {'value': v, 'unit': 'images/s', 'h2d_bytes_per_step': 0, 'd2h_bytes_per_step': 0}}
     print(json.dumps(line), flush=True)
 
@@ -326,6 +334,14 @@ def run_ours(args, wl):
     ms_dev_local = timed.local_ms
     launches = eng.last_launch_count
     clocks = sampler.finish() if sampler else None
+    if args.dump_outputs and rank == 0:     # the last timed step's results, before later passes overwrite them
+        dump = {k: t.cpu().numpy() for k, t in
+                (('boxes', boxes), ('scores', scores), ('labels', labels), ('counts', counts))}
+        for i, k in enumerate(dump['counts']):      # rows past an image's count carry no detection
+            dump['boxes'][i, k:] = 0
+            dump['scores'][i, k:] = 0
+            dump['labels'][i, k:] = 0
+        write_outputs(args.dump_outputs, dump)
     ms_e2e = timed(step_host, args.steps, max(3, args.warmup))
 
     # ---- per-kernel-category device time (events around our own kernels) for the roofline
@@ -437,6 +453,9 @@ def main():
     ap.add_argument('--per-gpu-batch', type=int, default=0,
                     help='override the workload batch (latency studies; the headline number uses the default)')
     ap.add_argument('--layers', action='store_true', help='add a per-conv-layer timing table to the JSON line')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='write the outputs of the last timed step (boxes, scores, labels, counts) as DIR/<name>.npy; '
+                         'the inputs depend only on the arguments, so two builds can be compared output for output')
     ap.add_argument('--ncu-unpiped', action='store_true', help='with --ncu-range: single-stream forward')
     ap.add_argument('--ncu-range', action='store_true',
                     help='run warm-up, then one step inside cudaProfilerStart/Stop (for ncu --profile-from-start off)')
